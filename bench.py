@@ -11,7 +11,7 @@ proof: witness table in, 1152-byte proof out.  `value` has the witness table res
 Second clause (configs[1]): a 2^20-point BN254 G1 MSM per GPU, reported in the `msm` object of the
 same JSON line as achieved GB/s of algorithmic bytes (96 B per (point, scalar) pair, SURVEY §8(d)).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--concurrency C]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--concurrency C] [--dump-outputs DIR]
 
 N > 1 (under torchrun, one rank per GPU): proofs are independent jobs — one proof stream per GPU,
 no data-path collective (weak scaling); the MSM leg shards one N*2^20-point MSM by point range
@@ -35,6 +35,7 @@ import time
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "examples"))  # host_circuits: caller-side restatement of the reference's circuits
 
@@ -101,6 +102,18 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx or None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_proof(out_dir, proof):
+    """`--dump-outputs`: one <field>.npy per field of the proof, float64.  Coordinates and evaluations are 256-bit
+    integers (Montgomery form, as the C ABI returns them); each is stored as its eight 32-bit little-endian words, which
+    float64 holds exactly, so two builds can be compared bit for bit: shape (..., 16) per G1 point, (..., 8) per Fr."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, _ in type(proof)._fields_:
+        limbs = np.ctypeslib.as_array(getattr(proof, name))
+        words = np.ascontiguousarray(limbs, dtype="<u8").view("<u4")
+        np.save(os.path.join(out_dir, name + ".npy"), words.astype(np.float64))
 
 
 def make_circuit(kind, log_n, seed):
@@ -170,7 +183,6 @@ def real_statement_leg(pool, ctx, d_srs_ptr, conc, steps, srs_host=None, cpu_bas
         if cpu_baseline:  # the oracle prover on the same tables, SRS and blinders — the only use of oracle/ in this leg
             sys.path.insert(0, os.path.join(ROOT, "oracle"))
             import oracle_c
-            oracle_c.build()
             oracle_c.autotune_threads()
             srs_np = srs_host[:circ.n + 3]
             opk = oracle_c.plonk_preprocess(circ.log_n, circ.selectors, circ.perm, circ.k, srs_np)
@@ -242,7 +254,6 @@ def private_match_bundle_leg(pool, ctx, d_srs_ptr, conc, bundles, srs_host=None,
     if cpu_baseline:
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import oracle_c
-        oracle_c.build()
         oracle_c.autotune_threads()
         srs_np = srs_host
         opks = [oracle_c.plonk_preprocess(c.log_n, c.selectors, c.perm, c.k, srs_np[:c.n + 3]) for c in circs]
@@ -368,7 +379,6 @@ def run_reference(args, rank, world):
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import oracle_c
     from renegade_b200 import synth
-    oracle_c.build()
     t0 = time.perf_counter()
     cores = oracle_c.autotune_threads()  # all logical CPUs unless a subset is faster on this (shared) host
     log_n = LOG_N
@@ -427,7 +437,12 @@ def main():
     ap.add_argument("--circuit", choices=("synthetic", "merkle"), default="synthetic",
                     help="synthetic: random gates of the reference's mix (default); merkle: height-10 Poseidon2 Merkle "
                          "openings built with the reference's gadgets (examples/host_circuits/circuit.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed proofs, write the last one (the proof a caller receives) to DIR as one "
+                         ".npy per field; the inputs depend on the arguments only, so two builds can be compared")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device prover's proof; the reference arm has none")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -529,6 +544,8 @@ def main():
     graph_launches = int(ctx._lib.b200_graph_launches() - graphs0)
     clocks = sampler.stop() if rank == 0 else None
     acc_tot = [c.msm_timing_totals(reset=True) for c in ctxs]
+    if args.dump_outputs and rank == 0:
+        dump_proof(args.dump_outputs, proof)  # the proof of the last timed step (blinders[warmup + steps - 1])
     # ---- the same through the public call with HOST buffers (e2e) ---------------------------------------
     run_proofs(2 * conc, h_wires.data_ptr(), 0)
     barrier()
@@ -780,7 +797,6 @@ def main():
     if not args.no_cpu_baseline and world == 1:
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import oracle_c  # CPU baseline leg: the only place the product arm executes the oracle
-        oracle_c.build()
         oracle_c.autotune_threads()
         h_srs = d_srs.cpu().numpy().view(np.uint64)
         opk = oracle_c.plonk_preprocess(LOG_N, circ.selectors, circ.perm, circ.k, h_srs)

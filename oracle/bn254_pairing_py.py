@@ -207,6 +207,43 @@ def decode_g2_mont(raw: bytes, i: int):
     return ((v[0], v[1]), (v[2], v[3]))
 
 
+def encode_g2_mont(pt) -> bytes:
+    """Inverse of decode_g2_mont: one 128-byte ptau G2 record."""
+    (x0, x1), (y0, y1) = pt
+    return b"".join((v * (1 << 256) % Q).to_bytes(32, "little") for v in (x0, x1, y0, y1))
+
+
+def g2_mul(pt, k: int):
+    """k * pt for an affine point of the twist (k > 0, k * pt not the identity), affine double-and-add over
+    Fq2 = Fq[u]/(u^2+1): builds [tau]_2 for an SRS whose tau is known."""
+    def mul(a, b):
+        return ((a[0] * b[0] - a[1] * b[1]) % Q, (a[0] * b[1] + a[1] * b[0]) % Q)
+
+    def sub(a, b):
+        return ((a[0] - b[0]) % Q, (a[1] - b[1]) % Q)
+
+    def inv(a):
+        d = pow((a[0] * a[0] + a[1] * a[1]) % Q, -1, Q)
+        return (a[0] * d % Q, -a[1] * d % Q)
+
+    def add(p1, p2):
+        (x1, y1), (x2, y2) = p1, p2
+        if x1 == x2:
+            assert y1 == y2, "P + (-P)"
+            m = mul(mul((3, 0), mul(x1, x1)), inv(mul((2, 0), y1)))
+        else:
+            m = mul(sub(y2, y1), inv(sub(x2, x1)))
+        x3 = sub(sub(mul(m, m), x1), x2)
+        return (x3, sub(mul(m, sub(x1, x3)), y1))
+
+    acc = None
+    for bit in bin(k)[2:]:
+        acc = None if acc is None else add(acc, acc)
+        if bit == "1":
+            acc = pt if acc is None else add(acc, pt)
+    return acc
+
+
 def g2_is_on_curve(pt) -> bool:
     """y^2 = x^3 + 3/(9+u) over Fq2 (the check srs.rs:193-194 makes)."""
     (x0, x1), (y0, y1) = pt

@@ -46,18 +46,26 @@ def srs_head():
         return f.read()
 
 
+PTAU_TAU = 0xB200B200B200
+
+
 @pytest.fixture(scope="session")
-def srs_2_16():
-    """The reference's own SRS, first 2^16 + 3 G1 powers (tests/golden/_large/srs_2_16.bin, cut by
-    tools/cut_srs_fixture.py from /root/reference/srs/srs00; git-ignored, ships with the gpurun snapshot)."""
-    path = os.path.join(ROOT, "tests", "golden", "_large", "srs_2_16.bin")
-    if not os.path.exists(path) and os.path.exists("/root/reference/srs/srs00"):
-        import subprocess
-        subprocess.check_call([sys.executable, os.path.join(ROOT, "tools", "cut_srs_fixture.py")])
-    if not os.path.exists(path):
-        pytest.skip("large SRS fixture absent (cut it where /root/reference exists: tools/cut_srs_fixture.py)")
-    with open(path, "rb") as f:
-        return f.read()
+def ptau_2_16(oracle, pyoracle, srs_head):
+    """A ptau file of 2^16 + 3 G1 powers of tau = PTAU_TAU: the 80-byte header of the reference's SRS file, then the
+    records [tau^i]_1.  The tests that prove circuits of up to 2^16 gates need that many powers; the reference's own
+    file is too large to store, so its first 512 powers and its G2 records are what tests/golden keeps of it."""
+    tau = oracle.int_to_limbs(pyoracle.to_mont(PTAU_TAU % pyoracle.R, pyoracle.R))
+    return srs_head[:80] + oracle.srs_from_tau(tau, (1 << 16) + 3).tobytes()
+
+
+@pytest.fixture(scope="session")
+def ptau_g2(g2_raw):
+    """(h, tau * h) of ptau_2_16: the reference's h and its multiple by PTAU_TAU, 16 x uint64 each."""
+    import numpy as np
+    import bn254_pairing_py as pr
+    h = g2_raw[0]
+    tau_h = pr.g2_mul(pr.decode_g2_mont(h.tobytes(), 0), PTAU_TAU)
+    return h, np.frombuffer(pr.encode_g2_mont(tau_h), dtype=np.uint64).copy()
 
 
 @pytest.fixture(scope="session")

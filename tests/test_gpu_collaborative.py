@@ -1,7 +1,7 @@
 """GPU parity of the collaborative prover (renegade_b200/collaborative.py on `DeviceBackend`: the C ABI's device-vector
 primitives, NTT and MSM): with 2 and 3 parties holding additive shares of the witness table and of the blinders, the opened
 proof is byte-identical to the device single-prover proof (`b200_plonk_prove`) and to the oracle's; then the
-`MultiProverCircuit` surface on the reference's own SRS: the VALID-MATCH-class settlement statement proved jointly by two
+`MultiProverCircuit` surface on a powers-of-tau SRS: the VALID-MATCH-class settlement statement proved jointly by two
 parties opens to a proof that the pairing verifier accepts under the single-prover circuit's verifying key
 (`multiprover_prove_and_verify`, circuits-core/src/lib.rs:166-177)."""
 import random
@@ -43,13 +43,13 @@ def test_device_collaborative_proof_equals_single_prover_proof(ctx, oracle, pyor
     pk.free()
 
 
-def test_multiprover_surface_on_the_reference_srs(ctx, srs_2_16, g2_raw):
+def test_multiprover_surface_on_the_reference_srs(ctx, ptau_2_16, ptau_g2):
     import renegade_b200 as rb
     from host_circuits import private_settlement as ps
     from host_circuits import statements as st
     from renegade_b200 import circuit_types as ct
-    h, tau_h = g2_raw
-    params = rb.parse_ptau_file(ctx, srs_2_16, count=(1 << 13) + 3)
+    h, tau_h = ptau_g2
+    params = rb.parse_ptau_file(ctx, ptau_2_16, count=(1 << 13) + 3)
     ct.set_system_srs(ctx, params.powers_of_g, h, tau_h)
     try:
         parties, statement = ps.create_witness_statement(seed=33)

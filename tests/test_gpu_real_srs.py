@@ -1,8 +1,8 @@
-"""GPU parity on the REFERENCE'S OWN SRS at the BASELINE size: the device prover commits against the first 2^16 + 3 powers
-of /root/reference/srs/srs00 (tests/golden/_large/srs_2_16.bin) and the proof must pass the pairing check against the
-file's own [tau]_2 — unknown tau, so nothing but a correct KZG opening passes — with the product verifier
-(`b200_plonk_verify`, host pairing) and with the independent pure-Python pairing of the oracle.  Then the
-`SingleProverCircuit` surface end to end on the real SRS: the restated reference statements prove, verify and link the
+"""GPU parity on a powers-of-tau SRS at the BASELINE size: the device prover commits against 2^16 + 3 powers read from a
+ptau file in the reference's layout (conftest `ptau_2_16`; the reference's own powers are pinned at n = 2^8 by
+test_pairing.py) and the proof must pass the pairing check against the matching [tau]_2 — the prover never sees tau, so
+nothing but a correct KZG opening passes — with the product verifier (`b200_plonk_verify`, host pairing) and with the
+independent pure-Python pairing of the oracle.  Then the `SingleProverCircuit` surface end to end on the same SRS: the restated reference statements prove, verify and link the
 way circuits-core's own tests do (`singleprover_prove_and_verify`, proof_linking/*.rs prove -> link -> verify)."""
 import random
 
@@ -13,16 +13,16 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.fixture(scope="module")
-def real_srs(ctx, srs_2_16):
+def real_srs(ctx, ptau_2_16):
     import renegade_b200 as rb
-    params = rb.parse_ptau_file(ctx, srs_2_16, count=(1 << 16) + 3)
+    params = rb.parse_ptau_file(ctx, ptau_2_16, count=(1 << 16) + 3)
     return params.powers_of_g
 
 
-def test_2_16_proof_on_the_reference_srs_passes_the_pairing_check(ctx, oracle, real_srs, g2_raw):
+def test_2_16_proof_on_the_reference_srs_passes_the_pairing_check(ctx, oracle, real_srs, ptau_g2):
     from renegade_b200 import synth
     from renegade_b200.backend import PlonkKzgSnark, VerifyingKey
-    h, tau_h = g2_raw
+    h, tau_h = ptau_g2
     log_n = 16
     circ = synth.synth_circuit(log_n, num_inputs=17, seed=0xB200, check=False)
     pk = PlonkKzgSnark.preprocess(ctx, real_srs, log_n, circ.num_inputs, circ.selectors, circ.perm, circ.k)
@@ -47,14 +47,14 @@ def test_2_16_proof_on_the_reference_srs_passes_the_pairing_check(ctx, oracle, r
     pk.free()
 
 
-def test_single_prover_circuit_surface_on_the_reference_srs(ctx, real_srs, g2_raw):
+def test_single_prover_circuit_surface_on_the_reference_srs(ctx, real_srs, ptau_g2):
     """circuits-core's own test shape: `singleprover_prove_and_verify::<C>(witness, statement)` for the restated
     statements, keys from the cache keyed by `C::name()` (traits.rs:1187-1201 checks the sharing), a wrong statement is
     refused by the verifier, an unsatisfied witness by the prover."""
     from host_circuits import statements as st
     from host_circuits import valid_balance_create as vbc
     from renegade_b200 import circuit_types as ct
-    h, tau_h = g2_raw
+    h, tau_h = ptau_g2
     ct.set_system_srs(ctx, real_srs, h, tau_h)
     try:
         w, s = vbc.create_witness_statement(7)
@@ -76,17 +76,17 @@ def test_single_prover_circuit_surface_on_the_reference_srs(ctx, real_srs, g2_ra
         ct.clear_key_cache()
 
 
-def test_private_match_bundle_through_the_surface(ctx, real_srs, g2_raw):
+def test_private_match_bundle_through_the_surface(ctx, real_srs, ptau_g2):
     """Prove -> link -> verify for one private match (native_proof_manager.rs:526-584, 726-782) with the typed surface:
     two INTENT AND BALANCE VALIDITY, two OUTPUT BALANCE VALIDITY and the PRIVATE SETTLEMENT proof, the four link proofs,
-    everything checked with the pairing against the reference's [tau]_2."""
+    everything checked with the pairing against the SRS's [tau]_2."""
     from host_circuits import intent_and_balance_validity as val
     from host_circuits import output_balance_validity as obv
     from host_circuits import private_settlement as ps
     from host_circuits import statements as st
     from renegade_b200 import circuit_types as ct
     from renegade_b200.backend import GroupLayout, link_proofs, verify_link_proof
-    h, tau_h = g2_raw
+    h, tau_h = ptau_g2
     ct.set_system_srs(ctx, real_srs, h, tau_h)
     try:
         parties, _ = ps.create_witness_statement(seed=61)

@@ -1,7 +1,7 @@
 """GPU test of the prover service end to end (SURVEY.md §8(f) f3): a client replays the requests the reference's
 `ProofServiceClient` would send (prover_service_client.rs:186-205: POST JSON, basic auth `admin`), the service proves
-through the pool on the device, and the returned proofs / link proofs verify with the pairing against the reference's
-own SRS."""
+through the pool on the device, and the returned proofs / link proofs verify with the pairing against a powers-of-tau SRS
+in the reference's ptau layout."""
 import threading
 
 import numpy as np
@@ -10,7 +10,7 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 
-def test_prove_paths_over_http(srs_2_16, g2_raw):
+def test_prove_paths_over_http(ptau_2_16, ptau_g2):
     import renegade_b200 as rb
     from host_circuits import intent_and_balance_validity as val
     from host_circuits import output_balance_validity as obv
@@ -21,10 +21,10 @@ def test_prove_paths_over_http(srs_2_16, g2_raw):
     from renegade_b200 import circuit_types as ct
     from renegade_b200 import service as sv
     from renegade_b200.backend import GroupLayout, ProverPool, verify_link_proof
-    h, tau_h = g2_raw
+    h, tau_h = ptau_g2
     pool = ProverPool(0, workers=4)
     ctx = pool.context(0)
-    params = rb.parse_ptau_file(ctx, srs_2_16, count=(1 << 14) + 3)
+    params = rb.parse_ptau_file(ctx, ptau_2_16, count=(1 << 14) + 3)
     ct.set_system_srs(ctx, params.powers_of_g, h, tau_h, pool=pool)
     service = sv.ProverService(service_routes.routes(), password="pw", pool=pool)
     server = service.make_server("127.0.0.1", 0)
@@ -89,17 +89,17 @@ def test_prove_paths_over_http(srs_2_16, g2_raw):
         pool.close()
 
 
-def _serve(srs_2_16, g2_raw, flow):
-    """A prover service over a 3-worker pool on device 0 with the reference's SRS; `flow(client, service)` drives it."""
+def _serve(ptau_2_16, ptau_g2, flow):
+    """A prover service over a 3-worker pool on device 0 with a powers-of-tau SRS; `flow(client, service)` drives it."""
     import renegade_b200 as rb
     from host_circuits import service_routes
     from renegade_b200 import circuit_types as ct
     from renegade_b200 import service as sv
     from renegade_b200.backend import ProverPool
-    h, tau_h = g2_raw
+    h, tau_h = ptau_g2
     pool = ProverPool(0, workers=3)
     ctx = pool.context(0)
-    params = rb.parse_ptau_file(ctx, srs_2_16, count=(1 << 14) + 3)
+    params = rb.parse_ptau_file(ctx, ptau_2_16, count=(1 << 14) + 3)
     ct.set_system_srs(ctx, params.powers_of_g, h, tau_h, pool=pool)
     service = sv.ProverService(service_routes.routes(), password="pw", pool=pool)
     server = service.make_server("127.0.0.1", 0)
@@ -112,25 +112,25 @@ def _serve(srs_2_16, g2_raw, flow):
         pool.close()
 
 
-def test_state_update_paths_over_http(srs_2_16, g2_raw):
+def test_state_update_paths_over_http(ptau_2_16, ptau_g2):
     """VALID DEPOSIT, VALID WITHDRAWAL, VALID ORDER CANCELLATION, VALID NOTE REDEMPTION and the two PUBLIC fee payments
     (`ProofResponse` paths, prover_service_client.rs:101-147) through the service on the device: the proofs verify with the
     pairing under the circuits' cached keys; a request whose statement does not belong to its witness comes back as a
     prover error.  (The same flow runs on the CPU with the oracle prover in tests/test_service_flows_cpu.py.)"""
     import service_flows
-    _serve(srs_2_16, g2_raw, service_flows.plain_proof_paths)
+    _serve(ptau_2_16, ptau_g2, service_flows.plain_proof_paths)
 
 
-def test_intent_only_paths_over_http(srs_2_16, g2_raw):
+def test_intent_only_paths_over_http(ptau_2_16, ptau_g2):
     """The intent-only flow as the relayer drives it: INTENT ONLY VALIDITY and FIRST FILL VALIDITY (`ProofAndHintResponse`),
     then INTENT ONLY PUBLIC / BOUNDED SETTLEMENT with the validity proof's hint (`SettlementProofResponse {proof, link_proof}`,
     api_types.rs:97-104, 279-299); link proofs between circuits of 2^13 / 2^11 and 2^9 rows verify with the pairing."""
     import service_flows
-    _serve(srs_2_16, g2_raw, lambda client, service: service_flows.intent_only_flow(client, service, g2_raw))
+    _serve(ptau_2_16, ptau_g2, lambda client, service: service_flows.intent_only_flow(client, service, ptau_g2))
 
 
-def test_public_settlement_paths_over_http(srs_2_16, g2_raw):
+def test_public_settlement_paths_over_http(ptau_2_16, ptau_g2):
     """INTENT AND BALANCE PUBLIC / BOUNDED SETTLEMENT with the party's validity and output-balance hints
     (`PublicSettlementProofResponse`, api_types.rs:126-137, 238-277)."""
     import service_flows
-    _serve(srs_2_16, g2_raw, lambda client, service: service_flows.public_settlement_flow(client, service, g2_raw))
+    _serve(ptau_2_16, ptau_g2, lambda client, service: service_flows.public_settlement_flow(client, service, ptau_g2))

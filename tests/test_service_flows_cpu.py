@@ -1,5 +1,5 @@
 """CPU: the prover service's request flows for the later statements, end to end — HTTP, codec, routing, the
-`SingleProverCircuit` surface with its key cache, link proofs, and the product's pairing verifier on the reference's own
+`SingleProverCircuit` surface with its key cache, link proofs, and the product's pairing verifier on a powers-of-tau
 SRS — with the ORACLE prover standing in for the device (test infrastructure: the device prover is byte-identical to it,
 tests/test_gpu_plonk.py).  The very same flows run against the device in tests/test_gpu_service.py."""
 import threading
@@ -44,12 +44,12 @@ def _oracle_snark(oracle):
 
 
 @pytest.fixture()
-def served(oracle, srs_2_16, g2_raw, monkeypatch):
+def served(oracle, ptau_2_16, ptau_g2, monkeypatch):
     """(client, service): the product's service + routes + circuit surface, the oracle where the device would prove."""
     from host_circuits import service_routes
-    h, tau_h = g2_raw
+    h, tau_h = ptau_g2
     n_srs = (1 << 14) + 3
-    srs = np.frombuffer(srs_2_16[80:80 + 64 * n_srs], dtype=np.uint64).reshape(n_srs, 8).copy()
+    srs = np.frombuffer(ptau_2_16[80:80 + 64 * n_srs], dtype=np.uint64).reshape(n_srs, 8).copy()
     monkeypatch.setattr(ct, "PlonkKzgSnark", _oracle_snark(oracle))
 
     def link_proofs(ctx, bases, a, b, layout):
@@ -75,16 +75,16 @@ def test_plain_proof_paths(served):
     service_flows.plain_proof_paths(*served, negatives="first")
 
 
-def test_intent_only_flow(served, g2_raw):
-    service_flows.intent_only_flow(*served, g2_raw)
+def test_intent_only_flow(served, ptau_g2):
+    service_flows.intent_only_flow(*served, ptau_g2)
 
 
-def test_public_settlement_flow(served, g2_raw):
-    service_flows.public_settlement_flow(*served, g2_raw, which=("public",))
+def test_public_settlement_flow(served, ptau_g2):
+    service_flows.public_settlement_flow(*served, ptau_g2, which=("public",))
 
 
-def test_private_match_flow(served, g2_raw):
-    service_flows.private_match_flow(*served, g2_raw)
+def test_private_match_flow(served, ptau_g2):
+    service_flows.private_match_flow(*served, ptau_g2)
 
 
 def test_structure_fingerprint_guards_the_key_cache(served, monkeypatch):
