@@ -238,6 +238,51 @@ int b200_plonk_verify_link(const uint64_t* comm1, const uint64_t* comm2, unsigne
  * (srs.rs:236-266: e(tau^i G, tau H) == e(tau^(i+1) G, H)). */
 int b200_pairing_check(const uint64_t* g1_points, const uint64_t* g2_points, size_t k, int* is_one);
 
+/* ---- batch verification (device) --------------------------------------------------------------
+ * Many PlonK proofs and link proofs checked in one call: the per-item work (on-curve checks, transcript replay, scalar
+ * algebra, the G1 operands of each item's KZG check e(A_j, [tau]_2) == e(B_j, [1]_2)) runs on the context's device; the
+ * items are folded with the powers of a Fiat–Shamir weight rho (a Keccak challenge over every item's final transcript
+ * state, each link item's opening proof and group layout, and the two G2 records) into ONE two-pair pairing product on
+ * the host.  Upstream jellyfish has `PlonkKzgSnark::batch_verify` for this use; the scheme here is this library's own.
+ * Verdicts are exactly those of the single verifiers above. */
+/* One verifying key of a batch: the flat key of b200_plonk_verify. */
+typedef struct {
+    unsigned log_n;
+    size_t num_inputs;
+    const uint64_t* k;              /* 5 x 4 limbs */
+    const uint64_t* selector_comms; /* 13 x 8 limbs */
+    const uint64_t* sigma_comms;    /* 5 x 8 limbs */
+} b200_batch_vk;
+/* One PlonK proof of a batch, checked against vks[vk] with num_inputs public inputs. */
+typedef struct {
+    unsigned vk;
+    const uint64_t* pub_inputs;
+    size_t num_inputs;
+    const b200_proof* proof;
+} b200_batch_proof;
+/* One link proof of a batch: the arguments of b200_plonk_verify_link. */
+typedef struct {
+    const uint64_t* comm1;
+    const uint64_t* comm2;
+    unsigned alignment;
+    size_t offset;
+    size_t size;
+    const b200_link_proof* proof;
+} b200_batch_link;
+/* *accepted = 1 exactly when every proof and link proof verifies.  item_accepted (may be NULL): n_proofs + n_links
+ * flags, proofs first, each equal to what b200_plonk_verify / b200_plonk_verify_link returns for that item alone (an
+ * off-curve element, an off-curve key point, or a public-input count other than the key's is a 0, not an error); when
+ * the combined check fails, contiguous ranges of items are bisected with the same weights, at most about
+ * 2 k log2(n) pairing products for k bad items.  operands (may be NULL): per item the unweighted (A_j, B_j), 2 x 8
+ * limbs, affine Montgomery, the identity as zeros (also for an item rejected before its check).
+ * pairing_products (may be NULL): how many pairing products the call evaluated.
+ * B200_ERR_INVALID: a NULL where data is required, vk >= n_vks, log_n > 28, alignment > 28, size == 0 or an empty
+ * batch; B200_ERR_NOT_ON_CURVE: an off-curve G2 point.  Synchronous, on the context's stream; keeps no pointer. */
+int b200_plonk_batch_verify(b200_ctx* ctx, const b200_batch_vk* vks, size_t n_vks, const b200_batch_proof* proofs,
+                            size_t n_proofs, const b200_batch_link* links, size_t n_links, const uint64_t g2_h[16],
+                            const uint64_t g2_tau_h[16], int* accepted, uint8_t* item_accepted, uint64_t* operands,
+                            size_t* pairing_products);
+
 /* Wall-clock milliseconds of the last proof's phases on this context: round 1, round 2, round 3
  * (coset NTTs + quotient + split), round 3 commitments, round 4, round 5, then two spare slots. */
 int b200_plonk_last_timings(b200_ctx* ctx, float out_ms[8]);

@@ -23,7 +23,7 @@ EXPORTS = [
     "b200_ntt", "b200_ntt_device", "b200_ntt_last_ms", "b200_domain_generator",
     "b200_splitmix_fr_device", "b200_known_dlog_bases_device",
     "b200_selftest_field", "b200_field_op",
-    "b200_plonk_preprocess", "b200_pk_verifying_key", "b200_pk_num_inputs", "b200_pk_log_n", "b200_pk_free", "b200_plonk_prove", "b200_plonk_link", "b200_plonk_verify", "b200_plonk_verify_link", "b200_pairing_check", "b200_plonk_last_timings", "b200_keccak256",
+    "b200_plonk_preprocess", "b200_pk_verifying_key", "b200_pk_num_inputs", "b200_pk_log_n", "b200_pk_free", "b200_plonk_prove", "b200_plonk_link", "b200_plonk_verify", "b200_plonk_verify_link", "b200_plonk_batch_verify", "b200_pairing_check", "b200_plonk_last_timings", "b200_keccak256",
     "b200_fr_vec_op", "b200_fr_batch_inverse_device", "b200_fr_poly_eval_device", "b200_fr_poly_div_linear_device",
     "b200_poseidon2_hash_batch", "b200_poseidon2_permute_batch", "b200_poseidon2_merkle_root_batch", "b200_poseidon2_csprng_batch",
     "b200_pool_create", "b200_pool_destroy", "b200_pool_workers", "b200_pool_ctx", "b200_pool_submit_prove",
@@ -106,6 +106,7 @@ def load() -> C.CDLL:
     lib.b200_plonk_link.argtypes = [vp, vp, vp, sz, vp, sz, vp, vp, u32, sz, sz, vp, vp]
     lib.b200_plonk_verify.argtypes = [u32, sz, vp, vp, vp, vp, vp, vp, vp, C.POINTER(i32)]
     lib.b200_plonk_verify_link.argtypes = [vp, vp, u32, sz, sz, vp, vp, vp, C.POINTER(i32)]
+    lib.b200_plonk_batch_verify.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, vp, C.POINTER(i32), vp, vp, C.POINTER(sz)]
     lib.b200_pairing_check.argtypes = [vp, vp, sz, C.POINTER(i32)]
     lib.b200_plonk_last_timings.argtypes = [vp, C.POINTER(C.c_float * 8)]
     lib.b200_fr_vec_op.argtypes = [vp, i32, vp, vp, i32, sz, vp]

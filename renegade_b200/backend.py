@@ -397,6 +397,58 @@ class PlonkKzgSnark:
         return bool(ok.value)
 
     @staticmethod
+    def batch_verify(ctx: Context, vks, public_inputs, proofs, links=(), want_operands: bool = False, g2=None):
+        """Verifies many proofs and link proofs on the device with one pairing product (`b200_plonk_batch_verify`).
+
+        vks[i], public_inputs[i], proofs[i] describe proof i; links are (comm_a, comm_b, B200LinkProof, GroupLayout).
+        Returns a numpy bool array of per-item verdicts, proofs first, each what `verify` / `verify_link_proof` says
+        for that item alone (a wrong public-input count is False).  With want_operands, also the (n, 2, 8) uint64 array
+        of each item's unweighted pairing operands (A_j, B_j).  The G2 pair (h, beta_h) comes from the verifying keys,
+        which must agree on it, or from `g2` for a batch of link proofs only.  `ctx` runs the device work: give the verifier a context of its own (not a prover pool worker's)."""
+        vks, public_inputs, proofs, links = list(vks), list(public_inputs), list(proofs), list(links)
+        if not (len(vks) == len(public_inputs) == len(proofs)):
+            raise ValueError("vks, public_inputs and proofs must have the same length")
+        if not vks and not links:
+            raise ValueError("empty batch")
+        if vks:
+            g2_h, g2_tau_h = _u64(vks[0].g2_h, (16,)), _u64(vks[0].g2_tau_h, (16,))
+        elif g2 is not None:
+            g2_h, g2_tau_h = _u64(g2[0], (16,)), _u64(g2[1], (16,))
+        else:
+            raise ValueError("a batch of link proofs only needs the G2 pair: pass g2=(h, beta_h)")
+        keep = []  # every array whose address goes into the call stays referenced here until it returns
+        table, index = [], {}
+        for vk in vks:
+            if not (np.array_equal(_u64(vk.g2_h, (16,)), g2_h) and np.array_equal(_u64(vk.g2_tau_h, (16,)), g2_tau_h)):
+                raise ValueError("verifying keys of one batch must share the G2 elements")
+            if id(vk) not in index:
+                index[id(vk)] = len(table)
+                arrs = (_u64(vk.k, (5, 4)), _u64(vk.selector_comms, (13, 8)), _u64(vk.sigma_comms, (5, 8)))
+                keep.append(arrs)
+                table.append(B200BatchVk(vk.log_n, vk.num_inputs, *(_ptr(a) for a in arrs)))
+        bp = (B200BatchProof * len(proofs))()
+        for i, (vk, pi, proof) in enumerate(zip(vks, public_inputs, proofs)):
+            pia = _u64(pi, (-1, 4))
+            keep.append(pia)
+            bp[i] = B200BatchProof(index[id(vk)], _ptr(pia) if pia.size else None, pia.shape[0], C.addressof(proof))
+        bl = (B200BatchLink * len(links))()
+        for i, (comm_a, comm_b, lp, layout) in enumerate(links):
+            ca, cb = _u64(comm_a, (8,)), _u64(comm_b, (8,))
+            keep.append((ca, cb))
+            bl[i] = B200BatchLink(_ptr(ca), _ptr(cb), layout.alignment, layout.offset, layout.size, C.addressof(lp))
+        vt = (B200BatchVk * len(table))(*table)
+        n = len(proofs) + len(links)
+        flags = np.zeros(n, dtype=np.uint8)
+        ops = np.zeros((n, 2, 8), dtype=np.uint64) if want_operands else None
+        ok = C.c_int(0)
+        _lib.check(ctx._lib.b200_plonk_batch_verify(ctx._h, vt, len(table), bp, len(proofs), bl if links else None, len(links),
+                                                    _ptr(g2_h), _ptr(g2_tau_h), C.byref(ok),
+                                                    flags.ctypes.data_as(C.c_void_p),
+                                                    _ptr(ops) if want_operands else None, None))
+        verdicts = flags.astype(bool)
+        return (verdicts, ops) if want_operands else verdicts
+
+    @staticmethod
     def preprocess(ctx: Context, srs: Bases, log_n: int, num_inputs: int, selectors: np.ndarray,
                    perm: np.ndarray, k: np.ndarray) -> ProvingKey:
         sel = np.ascontiguousarray(selectors, dtype=np.uint64).reshape(13, 1 << log_n, 4)
@@ -456,6 +508,23 @@ class B200LinkProof(C.Structure):
 
     def to_array(self) -> np.ndarray:
         return np.frombuffer(bytes(self), dtype=np.uint64).copy()
+
+
+class B200BatchVk(C.Structure):
+    """b200_batch_vk: one verifying key of a batch (the flat key of b200_plonk_verify)."""
+    _fields_ = [("log_n", C.c_uint), ("num_inputs", C.c_size_t), ("k", C.c_void_p), ("selector_comms", C.c_void_p),
+                ("sigma_comms", C.c_void_p)]
+
+
+class B200BatchProof(C.Structure):
+    """b200_batch_proof: one PlonK proof of a batch against key `vk` of the batch's key table."""
+    _fields_ = [("vk", C.c_uint), ("pub_inputs", C.c_void_p), ("num_inputs", C.c_size_t), ("proof", C.c_void_p)]
+
+
+class B200BatchLink(C.Structure):
+    """b200_batch_link: one link proof of a batch (the arguments of b200_plonk_verify_link)."""
+    _fields_ = [("comm1", C.c_void_p), ("comm2", C.c_void_p), ("alignment", C.c_uint), ("offset", C.c_size_t),
+                ("size", C.c_size_t), ("proof", C.c_void_p)]
 
 
 @dataclass

@@ -227,6 +227,9 @@ struct Context {
     int use_graphs = -1;  // 1 / 0: replay prover rounds as CUDA graphs or not; -1: B200_GRAPHS from the environment (default on)
     std::vector<ProofGraphSet*> graph_sets;
     uint64_t graph_clock = 0;
+    // batch verifier (batch_verify.cu): device workspace and the pinned staging of its inputs and results
+    DevBuf bv_dev;
+    HostPinned bv_host;
     ~Context();
 };
 

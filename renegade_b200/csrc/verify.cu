@@ -19,13 +19,16 @@
 //     final exponentiation split into the easy part (q^6 - 1)(q^2 + 1) and the hard part by the x-addition chain of
 //     Fuentes-Castaneda et al. (three exponentiations by x and Frobenius maps).
 // Clarity first: flat Fq12 arithmetic, affine Miller steps; a verification is ~6 ms of host time.
+// The transcript replay and the scalar assembly are verify_algebra.cuh's (shared with the device batch verifier,
+// batch_verify.cu, which also calls the pairing below through pairing.h).
 #include <cstring>
 #include <mutex>
 #include <vector>
 
 #include "b200prover.h"
 #include "device_ctx.h"
-#include "transcript.h"
+#include "pairing.h"
+#include "verify_algebra.cuh"
 
 namespace b200 {
 
@@ -34,10 +37,7 @@ namespace {
 using Fq = FqCfg;
 using Fr = FrCfg;
 
-// ---- Fq2 = Fq[u] / (u^2 + 1) ---------------------------------------------------------------------------
-struct fq2 {
-    fe a, b;  // a + b u
-};
+// ---- Fq2 = Fq[u] / (u^2 + 1) (struct fq2 in pairing.h) -----------------------------------------------------
 inline fq2 fq2_add(const fq2& x, const fq2& y) { return {fe_add<Fq>(x.a, y.a), fe_add<Fq>(x.b, y.b)}; }
 inline fq2 fq2_sub(const fq2& x, const fq2& y) { return {fe_sub<Fq>(x.a, y.a), fe_sub<Fq>(x.b, y.b)}; }
 inline fq2 fq2_neg(const fq2& x) { return {fe_neg<Fq>(x.a), fe_neg<Fq>(x.b)}; }
@@ -54,11 +54,6 @@ inline fq2 fq2_inv(const fq2& x) {  // 1 / (a + b u) = (a - b u) / (a^2 + b^2)
 }
 inline bool fq2_is_zero(const fq2& x) { return fe_is_zero(x.a) && fe_is_zero(x.b); }
 inline bool fq2_eq(const fq2& x, const fq2& y) { return fe_eq(x.a, y.a) && fe_eq(x.b, y.b); }
-
-struct g2_affine {
-    fq2 x, y;
-    bool inf;
-};
 
 // ---- Fq12 = Fq[w] / (w^12 - 18 w^6 + 82), flat coefficients -----------------------------------------------
 struct fq12 {
@@ -371,6 +366,46 @@ fq12 final_exponentiation(const fq12& f) {
     return fq12_mul(fq12_frob1(fq12_frob2(y15)), y14);  // q^3 = q o q^2
 }
 
+// ---- G1 sums of the host verifiers (host XYZZ arithmetic of ec.cuh) ----------------------------------------
+// sum_i s_i P_i over a term list, evaluated with ONE chain of doublings (Straus: 254 doublings in all and a mixed
+// addition per set scalar bit, instead of 254 doublings per term)
+g1_affine g1_sum_terms(const G1Term* terms, int n) {
+    std::vector<g1_affine> pts;
+    std::vector<fe> scalars;  // canonical (non-Montgomery) limbs
+    for (int i = 0; i < n; ++i) {
+        if (g1_affine_is_inf(terms[i].p) || fe_is_zero(terms[i].s)) continue;
+        pts.push_back(terms[i].p);
+        scalars.push_back(fe_from_mont<Fr>(terms[i].s));
+    }
+    g1_xyzz acc = g1_xyzz_inf();
+    for (int bit = 253; bit >= 0; --bit) {
+        acc = g1_dbl(acc);
+        for (size_t i = 0; i < pts.size(); ++i)
+            if ((scalars[i].l[bit >> 5] >> (bit & 31)) & 1u) acc = g1_add_mixed(acc, pts[i]);
+    }
+    return g1_to_affine(acc);
+}
+
+g1_affine g1_load(const uint64_t xy[8]) {
+    g1_affine p;
+    std::memcpy(&p, xy, 64);
+    return p;
+}
+
+// e(A, [tau]_2) == e(B, [1]_2)   <=>   e(A, [tau]_2) * e(-B, [1]_2) == 1
+int check_operands(const OperandTerms& t, const uint64_t g2_h[16], const uint64_t g2_tau_h[16], const char* who, int* accepted) {
+    const g1_affine ps[2] = {g1_sum_terms(t.a, t.na), g1_affine_neg(g1_sum_terms(t.b, t.nb))};
+    const g2_affine qs[2] = {g2_load(g2_tau_h), g2_load(g2_h)};
+    if (!g2_on_curve(qs[0]) || !g2_on_curve(qs[1])) {
+        set_error(std::string(who) + ": G2 point not on curve");
+        return B200_ERR_NOT_ON_CURVE;
+    }
+    *accepted = pairing_product_is_one(ps, qs, 2) ? 1 : 0;
+    return B200_OK;
+}
+
+}  // namespace
+
 bool g2_on_curve(const g2_affine& p) {
     if (p.inf) return true;
     // b' = 3 / (9 + u) = 3 (9 - u) / 82
@@ -379,7 +414,6 @@ bool g2_on_curve(const g2_affine& p) {
     return fq2_eq(fq2_sqr(p.y), fq2_add(fq2_mul(fq2_sqr(p.x), p.x), b));
 }
 
-// 128-byte record x0 || x1 || y0 || y1 (Montgomery), the ptau layout read by srs.rs:185-199
 g2_affine g2_load(const uint64_t rec[16]) {
     g2_affine p;
     std::memcpy(&p.x.a, rec, 32);
@@ -389,62 +423,10 @@ g2_affine g2_load(const uint64_t rec[16]) {
     p.inf = fq2_is_zero(p.x) && fq2_is_zero(p.y);
     return p;
 }
-g1_affine g1_load(const uint64_t xy[8]) {
-    g1_affine p;
-    std::memcpy(&p, xy, 64);
-    return p;
-}
-
-// ---- G1 helpers of the verifier (host XYZZ arithmetic of ec.cuh) -------------------------------------------
-// sum_i s_i P_i, collected first and evaluated with ONE chain of doublings (Straus: 254 doublings in all and a mixed
-// addition per set scalar bit, instead of 254 doublings per term)
-struct G1Sum {
-    std::vector<g1_affine> pts;
-    std::vector<fe> scalars;  // canonical (non-Montgomery) limbs
-    g1_xyzz eval() const {
-        g1_xyzz acc = g1_xyzz_inf();
-        for (int bit = 253; bit >= 0; --bit) {
-            acc = g1_dbl(acc);
-            for (size_t i = 0; i < pts.size(); ++i)
-                if ((scalars[i].l[bit >> 5] >> (bit & 31)) & 1u) acc = g1_add_mixed(acc, pts[i]);
-        }
-        return acc;
-    }
-};
-void g1_acc(G1Sum* acc, const g1_affine& p, const fe& s_mont) {
-    if (g1_affine_is_inf(p) || fe_is_zero(s_mont)) return;
-    acc->pts.push_back(p);
-    acc->scalars.push_back(fe_from_mont<Fr>(s_mont));
-}
-inline fe fr_pow_u64(fe a, uint64_t e) {
-    fe r = fe_one<Fr>();
-    while (e) {
-        if (e & 1) r = fe_mul<Fr>(r, a);
-        a = fe_sqr<Fr>(a);
-        e >>= 1;
-    }
-    return r;
-}
-
-constexpr int NW = 5, NS = 13;
-
-struct ProofIn {  // layout of b200_proof
-    g1_affine wires_poly_comms[NW];
-    g1_affine prod_perm_poly_comm;
-    g1_affine split_quot_poly_comms[NW];
-    g1_affine opening_proof;
-    g1_affine shifted_opening_proof;
-    fe wires_evals[NW];
-    fe wire_sigma_evals[NW - 1];
-    fe perm_next_eval;
-};
-static_assert(sizeof(ProofIn) == sizeof(b200_proof), "proof layout");
 
 bool pairing_product_is_one(const g1_affine* ps, const g2_affine* qs, size_t k) {
     return fq12_is_one(final_exponentiation(miller_loop_product(ps, qs, k)));
 }
-
-}  // namespace
 
 }  // namespace b200
 
@@ -478,130 +460,15 @@ int b200_plonk_verify(unsigned log_n, size_t num_inputs, const uint64_t* k, cons
         log_n > 28)
         return B200_ERR_INVALID;
     *accepted = 0;
-    const size_t n = (size_t)1 << log_n;
-    const ProofIn& proof = *reinterpret_cast<const ProofIn*>(proof_in);
-    const fe* kk = reinterpret_cast<const fe*>(k);
-    const g1_affine* sel = reinterpret_cast<const g1_affine*>(selector_comms);
-    const g1_affine* sig = reinterpret_cast<const g1_affine*>(sigma_comms);
-    const fe* pi = reinterpret_cast<const fe*>(pub_inputs);
-    // every group element the verifier multiplies must be on the curve (the identity is allowed)
-    {
-        bool ok = true;
-        for (int i = 0; i < NS; ++i) ok = ok && g1_affine_on_curve(sel[i]);
-        for (int i = 0; i < NW; ++i)
-            ok = ok && g1_affine_on_curve(sig[i]) && g1_affine_on_curve(proof.wires_poly_comms[i]) &&
-                 g1_affine_on_curve(proof.split_quot_poly_comms[i]);
-        ok = ok && g1_affine_on_curve(proof.prod_perm_poly_comm) && g1_affine_on_curve(proof.opening_proof) &&
-             g1_affine_on_curve(proof.shifted_opening_proof);
-        if (!ok) return B200_OK;  // rejected
-    }
-    // ---- challenges (same transcript as the prover, plonk.cu) ------------------------------------------------
-    SolidityTranscript tr;
-    tr.append_u32_be(254);
-    tr.append_u64_be((uint64_t)n);
-    tr.append_u64_be((uint64_t)num_inputs);
-    for (int i = 0; i < NW; ++i) tr.append_field_elem(kk[i]);
-    for (int s = 0; s < NS; ++s) tr.append_commitment(sel[s]);
-    for (int i = 0; i < NW; ++i) tr.append_commitment(sig[i]);
-    for (size_t i = 0; i < num_inputs; ++i) tr.append_field_elem(pi[i]);
-    for (int i = 0; i < NW; ++i) tr.append_commitment(proof.wires_poly_comms[i]);
-    const fe beta = tr.get_and_append_challenge();
-    const fe gamma = tr.get_and_append_challenge();
-    tr.append_commitment(proof.prod_perm_poly_comm);
-    const fe alpha = tr.get_and_append_challenge();
-    for (int i = 0; i < NW; ++i) tr.append_commitment(proof.split_quot_poly_comms[i]);
-    const fe zeta = tr.get_and_append_challenge();
-    for (int i = 0; i < NW; ++i) tr.append_field_elem(proof.wires_evals[i]);
-    for (int i = 0; i < NW - 1; ++i) tr.append_field_elem(proof.wire_sigma_evals[i]);
-    tr.append_field_elem(proof.perm_next_eval);
-    const fe v = tr.get_and_append_challenge();
-    tr.append_commitment(proof.opening_proof);
-    tr.append_commitment(proof.shifted_opening_proof);
-    const fe u = tr.get_and_append_challenge();
-
-    // ---- scalars ---------------------------------------------------------------------------------------------
-    const fe one = fe_one<Fr>();
-    const fe w = host_root_of_unity(log_n);
-    const fe vanish = fe_sub<Fr>(fr_pow_u64(zeta, (uint64_t)n), one);
-    fe nfr = fe_zero();
-    nfr.l[0] = (uint32_t)n;
-    nfr.l[1] = (uint32_t)((uint64_t)n >> 32);
-    nfr = fe_to_mont<Fr>(nfr);
-    // zeta on the domain makes L_1 / PI denominators vanish: the reference rejects such proofs too (probability ~ n / r)
-    const fe l1 = fe_mul<Fr>(vanish, fe_inv<Fr>(fe_mul<Fr>(fe_sub<Fr>(zeta, one), nfr)));
-    const fe alpha2 = fe_sqr<Fr>(alpha);
-    fe pi_eval = fe_zero(), wj = one;
-    for (size_t j = 0; j < num_inputs; ++j) {  // PI(zeta) = sum_j pi_j w^j Z_H(zeta) / (n (zeta - w^j))
-        fe t = fe_inv<Fr>(fe_mul<Fr>(fe_sub<Fr>(zeta, wj), nfr));
-        t = fe_mul<Fr>(fe_mul<Fr>(fe_mul<Fr>(t, vanish), wj), pi[j]);
-        pi_eval = fe_add<Fr>(pi_eval, t);
-        wj = fe_mul<Fr>(wj, w);
-    }
-    const fe* we = proof.wires_evals;
-    const fe* se = proof.wire_sigma_evals;
-    // r0 = PI - alpha^2 L1 - alpha z_w prod_{i<4} (w_i + beta s_i + gamma) (w_4 + gamma)
-    fe prod = fe_mul<Fr>(alpha, proof.perm_next_eval);
-    for (int j = 0; j < NW - 1; ++j) prod = fe_mul<Fr>(prod, fe_add<Fr>(fe_add<Fr>(fe_mul<Fr>(se[j], beta), we[j]), gamma));
-    const fe prod4 = fe_mul<Fr>(prod, fe_add<Fr>(we[4], gamma));
-    const fe r0 = fe_sub<Fr>(fe_sub<Fr>(pi_eval, fe_mul<Fr>(alpha2, l1)), prod4);
-
-    // ---- D: linearisation commitment ---------------------------------------------------------------------------
-    G1Sum D;  // F and B below only add terms to it: one evaluation at the end
-    auto pow5 = [](const fe& x) { return fe_mul<Fr>(fe_sqr<Fr>(fe_sqr<Fr>(x)), x); };
-    for (int j = 0; j < 4; ++j) g1_acc(&D, sel[j], we[j]);
-    g1_acc(&D, sel[4], fe_mul<Fr>(we[0], we[1]));
-    g1_acc(&D, sel[5], fe_mul<Fr>(we[2], we[3]));
-    for (int j = 0; j < 4; ++j) g1_acc(&D, sel[6 + j], pow5(we[j]));
-    g1_acc(&D, sel[10], fe_neg<Fr>(we[4]));
-    g1_acc(&D, sel[11], one);
-    g1_acc(&D, sel[12], fe_mul<Fr>(fe_mul<Fr>(fe_mul<Fr>(we[0], we[1]), fe_mul<Fr>(we[2], we[3])), we[4]));
-    fe coeff = alpha;
-    for (int j = 0; j < NW; ++j)
-        coeff = fe_mul<Fr>(coeff, fe_add<Fr>(fe_add<Fr>(fe_mul<Fr>(fe_mul<Fr>(kk[j], zeta), beta), we[j]), gamma));
-    coeff = fe_add<Fr>(coeff, fe_mul<Fr>(alpha2, l1));
-    g1_acc(&D, proof.prod_perm_poly_comm, coeff);
-    g1_acc(&D, sig[NW - 1], fe_neg<Fr>(fe_mul<Fr>(prod, beta)));
-    const fe zn2 = fe_mul<Fr>(fe_mul<Fr>(fe_add<Fr>(vanish, one), zeta), zeta);
-    fe c = fe_neg<Fr>(vanish);
-    for (int i = 0; i < NW; ++i) {
-        g1_acc(&D, proof.split_quot_poly_comms[i], c);
-        c = fe_mul<Fr>(c, zn2);
-    }
-    // ---- F, E: batched opening at zeta -------------------------------------------------------------------------
-    G1Sum& F = D;
-    fe E = fe_neg<Fr>(r0), vp = one;
-    for (int i = 0; i < NW; ++i) {
-        vp = fe_mul<Fr>(vp, v);
-        g1_acc(&F, proof.wires_poly_comms[i], vp);
-        E = fe_add<Fr>(E, fe_mul<Fr>(vp, we[i]));
-    }
-    for (int i = 0; i < NW - 1; ++i) {
-        vp = fe_mul<Fr>(vp, v);
-        g1_acc(&F, sig[i], vp);
-        E = fe_add<Fr>(E, fe_mul<Fr>(vp, se[i]));
-    }
-    // ---- pairing operands ----------------------------------------------------------------------------------------
-    g1_affine G;
-    G.x = fe_one<Fq>();
-    G.y = fe_from_u32<Fq>(2);
-    G1Sum A;
-    g1_acc(&A, proof.opening_proof, one);
-    g1_acc(&A, proof.shifted_opening_proof, u);
-    G1Sum& B = F;
-    g1_acc(&B, G, fe_neg<Fr>(E));
-    g1_acc(&B, proof.opening_proof, zeta);
-    g1_acc(&B, proof.shifted_opening_proof, fe_mul<Fr>(u, fe_mul<Fr>(zeta, w)));
-    g1_acc(&B, proof.prod_perm_poly_comm, u);
-    g1_acc(&B, G, fe_neg<Fr>(fe_mul<Fr>(u, proof.perm_next_eval)));
-    // e(A, [tau]_2) == e(B, [1]_2)   <=>   e(A, [tau]_2) * e(-B, [1]_2) == 1
-    const g1_affine ps[2] = {g1_to_affine(A.eval()), g1_affine_neg(g1_to_affine(B.eval()))};
-    const g2_affine qs[2] = {g2_load(g2_tau_h), g2_load(g2_h)};
-    if (!g2_on_curve(qs[0]) || !g2_on_curve(qs[1])) {
-        set_error("verify: G2 point not on curve");
-        return B200_ERR_NOT_ON_CURVE;
-    }
-    *accepted = pairing_product_is_one(ps, qs, 2) ? 1 : 0;
-    return B200_OK;
+    const VkIn vk = {reinterpret_cast<const fe*>(k), reinterpret_cast<const g1_affine*>(selector_comms),
+                     reinterpret_cast<const g1_affine*>(sigma_comms)};
+    std::vector<uint8_t> buf(plonk_transcript_bytes(num_inputs));
+    TranscriptT<ByteSpan> tr(ByteSpan{buf.data(), 0, buf.size()});
+    OperandTerms t;
+    if (!plonk_verify_terms(log_n, num_inputs, vk, reinterpret_cast<const fe*>(pub_inputs),
+                            *reinterpret_cast<const ProofIn*>(proof_in), host_root_of_unity(log_n), tr, &t))
+        return B200_OK;  // rejected
+    return check_operands(t, g2_h, g2_tau_h, "verify", accepted);
     B200_CATCH
 }
 
@@ -610,34 +477,13 @@ int b200_plonk_verify_link(const uint64_t* comm1, const uint64_t* comm2, unsigne
     B200_TRY
     if (!comm1 || !comm2 || !proof || !g2_h || !g2_tau_h || !accepted || alignment > 28 || size == 0) return B200_ERR_INVALID;
     *accepted = 0;
-    const g1_affine c1 = g1_load(comm1), c2 = g1_load(comm2);
-    const g1_affine cq = g1_load(proof->quotient_commitment), op = g1_load(proof->opening_proof);
-    if (!g1_affine_on_curve(c1) || !g1_affine_on_curve(c2) || !g1_affine_on_curve(cq) || !g1_affine_on_curve(op)) return B200_OK;
-    SolidityTranscript tr;
-    tr.append_commitment(c1);
-    tr.append_commitment(c2);
-    tr.append_commitment(cq);
-    const fe eta = tr.get_and_append_challenge();
-    const fe g = host_root_of_unity(alignment);
-    fe root = fr_pow_u64(g, (uint64_t)offset), zd = fe_one<Fr>();
-    for (size_t i = 0; i < size; ++i) {
-        zd = fe_mul<Fr>(zd, fe_sub<Fr>(eta, root));
-        root = fe_mul<Fr>(root, g);
-    }
-    // (tau - eta) pi == C1 - C2 - Z_D(eta) Cq   <=>   e(pi, [tau]_2) == e(C1 - C2 - Z_D(eta) Cq + eta pi, [1]_2)
-    G1Sum B;
-    g1_acc(&B, c1, fe_one<Fr>());
-    g1_acc(&B, g1_affine_neg(c2), fe_one<Fr>());
-    g1_acc(&B, cq, fe_neg<Fr>(zd));
-    g1_acc(&B, op, eta);
-    const g1_affine ps[2] = {op, g1_affine_neg(g1_to_affine(B.eval()))};
-    const g2_affine qs[2] = {g2_load(g2_tau_h), g2_load(g2_h)};
-    if (!g2_on_curve(qs[0]) || !g2_on_curve(qs[1])) {
-        set_error("verify_link: G2 point not on curve");
-        return B200_ERR_NOT_ON_CURVE;
-    }
-    *accepted = pairing_product_is_one(ps, qs, 2) ? 1 : 0;
-    return B200_OK;
+    uint8_t buf[kLinkTranscriptBytes];
+    TranscriptT<ByteSpan> tr(ByteSpan{buf, 0, sizeof(buf)});
+    OperandTerms t;
+    if (!link_verify_terms(g1_load(comm1), g1_load(comm2), g1_load(proof->quotient_commitment), g1_load(proof->opening_proof),
+                           host_root_of_unity(alignment), offset, size, tr, &t))
+        return B200_OK;  // rejected
+    return check_operands(t, g2_h, g2_tau_h, "verify_link", accepted);
     B200_CATCH
 }
 
