@@ -453,6 +453,71 @@ int b200_fr_poly_eval_device(b200_ctx* ctx, const void* d_coeffs, size_t len, co
 /* q = p / (X - z), remainder dropped (len - 1 coefficients written to d_q). */
 int b200_fr_poly_div_linear_device(b200_ctx* ctx, const void* d_p, size_t len, const uint64_t z[4], void* d_q);
 
+/* ---- collaborative prover (device) ------------------------------------------------------------
+ * `MultiproverPlonkKzgSnark::prove_with_link_hint(&circuit, &pk, fabric)` (traits.rs:1103-1154) for ONE party: each party
+ * calls b200_mpc_prove with its own context, its additive shares of the wire table and of the 17 blinders, its
+ * preprocessing and a transport to the other parties.  Every party returns the same opened proof and challenges, equal
+ * to b200_plonk_prove on the summed wire table and blinders; link_poly_share is this party's share of the linking
+ * polynomial (`MpcProofLinkingHint` stays shared).  Opened over the transport: the masked Beaver differences, the masked
+ * round-2 denominators den r, partial commitments (summed by the library), the five wire evaluations and z(zeta w), the
+ * quotient's coefficients above its degree (zero for a satisfied witness), one masked r q[deg], and the transcript state
+ * after the verifying key and the public inputs (every party must agree on it, else B200_ERR_INVALID everywhere).
+ * Shares are plain additive shares without MACs (semi-honest parties).
+ * Every message starts with a 32-byte header (exchange index, payload bytes, two zero words), checked on receipt: the
+ * wrong exchange or size is B200_ERR_INVALID.  Any failure after the argument checks calls transport->abort. */
+/* all_gather: send `bytes` bytes, receive every party's message in party order (parties * bytes, this party's
+ * included); return 0, or a negative code that aborts the proof.  abort (may be NULL): called when this party gives up,
+ * so that the others are not left waiting. */
+typedef struct {
+    int (*all_gather)(void* user, const void* mine, size_t bytes, void* all);
+    void (*abort)(void* user);
+    void* user;
+    int party;   /* 0 .. parties - 1; party 0 adds the public terms */
+    int parties; /* >= 2 */
+} b200_mpc_transport;
+/* Device-resident Beaver triples ([a], [b], [c = a b]) and masks for ONE proof; a second use is B200_ERR_INVALID
+ * (reused triples leak the witness).  Layout, n = 2^log_n, m = nc n with nc = 6 (8 below n = 16): round 2 takes
+ * R3 = 10 n + sum_{d = 1, 2, .., n/2} (n - d) triples, round 3 the next 26 m, the degree check the last one; the
+ * triples [R3 + 2m, R3 + 6m) and [R3 + 11m, R3 + 15m) are squares (c = a^2, b unused).  Masks: n + 1. */
+typedef struct b200_mpc_prep b200_mpc_prep;
+/* The exact numbers of triples and masks b200_mpc_prove consumes with this key. */
+int b200_mpc_prep_size(const b200_pk* pk, size_t* n_triples, size_t* n_masks);
+/* This party's shares from the caller's offline phase: a, b, c (n_triples x 4 limbs each), masks (n_masks x 4 limbs);
+ * host or device pointers, copied. */
+int b200_mpc_prep_load(b200_ctx* ctx, const b200_pk* pk, const uint64_t* a, const uint64_t* b, const uint64_t* c,
+                       const uint64_t* masks, b200_mpc_prep** out);
+/* INSECURE stand-in for the offline phase, for tests and benchmarks: party p's shares are derived on the device from
+ * (seed, p, parties) alone, so no exchange is needed; the last party computes the values and subtracts the other
+ * parties' shares.  Anyone who knows the seed knows every triple. */
+int b200_mpc_prep_dealer(b200_ctx* ctx, const b200_pk* pk, uint64_t seed, int party, int parties,
+                         b200_mpc_prep** out);
+void b200_mpc_prep_free(b200_ctx* ctx, b200_mpc_prep* prep);
+/* wire_shares: 5 x n (host or device pointer), pub_inputs: the key's num_inputs public values (the same on every party),
+ * blinder_shares: 17 (draw order of b200_plonk_prove), proof: the opened proof, link_poly_share (n + 2, may be NULL),
+ * challenges (6, may be NULL).  Parties on one device may pass the same key.  B200_ERR_UNSATISFIED on every party when
+ * the joint witness does not satisfy the circuit. */
+int b200_mpc_prove(b200_ctx* ctx, const b200_pk* pk, const b200_mpc_transport* transport, b200_mpc_prep* prep,
+                   const uint64_t* wire_shares, const uint64_t* pub_inputs, const uint64_t* blinder_shares,
+                   b200_proof* proof, uint64_t* link_poly_share, uint64_t* challenges);
+/* b200_plonk_link on shares of the two hints (a plaintext hint is passed as its holder's share, zeros elsewhere);
+ * comm1 / comm2 are the opened commitments.  Opens the interpolant's coefficients above len - 1 - size (zero when the
+ * hints agree on the group, else B200_ERR_UNSATISFIED on every party), the evaluation at eta and partial commitments.
+ * The result equals b200_plonk_link on the summed hints. */
+int b200_mpc_link(b200_ctx* ctx, const b200_bases* srs, const b200_mpc_transport* transport, const uint64_t* a1_share,
+                  size_t len1, const uint64_t* a2_share, size_t len2, const uint64_t* comm1, const uint64_t* comm2,
+                  unsigned alignment, size_t offset, size_t size, b200_link_proof* proof, uint64_t* eta);
+/* In-process all-gather between the threads of `parties` parties (one b200_mpc_prove call per thread).  After an
+ * abort, a failed all_gather or `timeout_ms` without the other parties, every pending and later all_gather of the group
+ * fails. */
+typedef struct b200_mpc_local_group b200_mpc_local_group;
+int b200_mpc_local_group_create(int parties, unsigned timeout_ms, b200_mpc_local_group** out);
+/* The transport of `party`; valid while the group lives. */
+int b200_mpc_local_group_transport(b200_mpc_local_group* group, int party, b200_mpc_transport* out);
+void b200_mpc_local_group_destroy(b200_mpc_local_group* group);
+/* The last b200_mpc_prove / b200_mpc_link on this context: exchanges, bytes sent (headers included), triples used,
+ * milliseconds inside all_gather. */
+int b200_mpc_last_stats(b200_ctx* ctx, double out[4]);
+
 /* ---- witness-side batch hashing (SURVEY.md §8(f) f4) ------------------------------------- */
 /* `batch` independent Poseidon2 sponge hashes of `len` scalars each (inputs: batch x len x 4
  * limbs, Montgomery; out: batch x 4 limbs; host or device pointers).  Each equals the reference's

@@ -35,6 +35,8 @@ EXPORTS = [
     "b200_nccl_version", "b200_multi_world", "b200_multi_local_devices", "b200_multi_ctx", "b200_multi_rank",
     "b200_multi_bases_load", "b200_multi_bases_known_dlog", "b200_multi_bases_free", "b200_multi_bases_len",
     "b200_multi_bases_shard", "b200_multi_bases_plan", "b200_multi_msm", "b200_multi_msm_local",
+    "b200_mpc_prep_size", "b200_mpc_prep_load", "b200_mpc_prep_dealer", "b200_mpc_prep_free", "b200_mpc_prove", "b200_mpc_link",
+    "b200_mpc_local_group_create", "b200_mpc_local_group_transport", "b200_mpc_local_group_destroy", "b200_mpc_last_stats",
 ]
 
 
@@ -170,6 +172,18 @@ def load() -> C.CDLL:
     lib.b200_multi_bases_plan.argtypes = [vp, i32, C.POINTER(i32 * 4)]
     lib.b200_multi_msm.argtypes = [vp, vp, vp, sz, i32, vp, C.POINTER(i32)]
     lib.b200_multi_msm_local.argtypes = [vp, vp, C.POINTER(vp), i32, i32, vp, C.POINTER(i32)]
+    lib.b200_mpc_prep_size.argtypes = [vp, C.POINTER(sz), C.POINTER(sz)]
+    lib.b200_mpc_prep_load.argtypes = [vp, vp, vp, vp, vp, vp, C.POINTER(vp)]
+    lib.b200_mpc_prep_dealer.argtypes = [vp, vp, u64, i32, i32, C.POINTER(vp)]
+    lib.b200_mpc_prep_free.argtypes = [vp, vp]
+    lib.b200_mpc_prep_free.restype = None
+    lib.b200_mpc_prove.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.b200_mpc_link.argtypes = [vp, vp, vp, vp, sz, vp, sz, vp, vp, u32, sz, sz, vp, vp]
+    lib.b200_mpc_local_group_create.argtypes = [i32, u32, C.POINTER(vp)]
+    lib.b200_mpc_local_group_transport.argtypes = [vp, i32, vp]
+    lib.b200_mpc_local_group_destroy.argtypes = [vp]
+    lib.b200_mpc_local_group_destroy.restype = None
+    lib.b200_mpc_last_stats.argtypes = [vp, C.POINTER(C.c_double * 4)]
     lib.b200_keccak256.argtypes = [C.c_char_p, sz, vp]
     lib.b200_keccak256.restype = None
     for name in EXPORTS:

@@ -525,3 +525,189 @@ class MultiproverPlonkKzgSnark:
         set_g1(proof.shifted_opening_proof, xy)
         hint = LinkingHint(linking_wire_poly=be.to_limbs(link_poly), linking_wire_comm=np.array(proof.wires_poly_comms[0], dtype=np.uint64))
         return proof, hint, fab
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# the protocol on the device: one party per call (b200_mpc_prove / b200_mpc_link)
+# ---------------------------------------------------------------------------------------------------------------
+ALL_GATHER = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p)
+ABORT = C.CFUNCTYPE(None, C.c_void_p)
+
+
+class MpcTransport(C.Structure):
+    """b200_mpc_transport: all_gather(user, mine, bytes, all) and abort(user) of one party."""
+    _fields_ = [("all_gather", ALL_GATHER), ("abort", ABORT), ("user", C.c_void_p), ("party", C.c_int), ("parties", C.c_int)]
+
+
+def callback_transport(party: int, parties: int, all_gather, abort=None) -> MpcTransport:
+    """A transport written in Python: `all_gather(mine: bytes) -> bytes` returns every party's message in party order
+    (or None / raises to fail the exchange); `abort()` is called when this party gives up."""
+    def _gather(_user, mine, nbytes, out):
+        try:
+            got = all_gather(C.string_at(mine, nbytes))
+        except Exception:
+            return -1
+        if got is None or len(got) != parties * nbytes:
+            return -1
+        C.memmove(out, got, len(got))
+        return 0
+
+    def _abort(_user):
+        if abort is not None:
+            abort()
+
+    t = MpcTransport(ALL_GATHER(_gather), ABORT(_abort), None, party, parties)
+    t._keep = (t.all_gather, t.abort)  # the C callbacks live as long as the structure
+    return t
+
+
+class LocalGroup:
+    """b200_mpc_local_group: an in-process all-gather between the threads of `parties` parties."""
+
+    def __init__(self, parties: int, timeout_ms: int = 120000):
+        self._lib = _lib.load()
+        self._h = C.c_void_p()
+        _lib.check(self._lib.b200_mpc_local_group_create(parties, timeout_ms, C.byref(self._h)))
+        self.parties = parties
+
+    def transport(self, party: int) -> MpcTransport:
+        t = MpcTransport()
+        _lib.check(self._lib.b200_mpc_local_group_transport(self._h, party, C.byref(t)))
+        return t
+
+    def close(self):
+        if self._h:
+            self._lib.b200_mpc_local_group_destroy(self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class MpcPrep:
+    """b200_mpc_prep: one party's Beaver triples and masks for ONE proof (device-resident, single-use)."""
+
+    def __init__(self, ctx: Context, handle):
+        self._ctx, self._h = ctx, handle
+
+    @staticmethod
+    def size(pk) -> tuple:
+        t, m = C.c_size_t(), C.c_size_t()
+        _lib.check(_lib.load().b200_mpc_prep_size(pk._h, C.byref(t), C.byref(m)))
+        return t.value, m.value
+
+    @staticmethod
+    def dealer(ctx: Context, pk, seed: int, party: int, parties: int) -> "MpcPrep":
+        """INSECURE stand-in for an offline phase (tests, benchmarks): shares derived from (seed, party, parties)."""
+        h = C.c_void_p()
+        _lib.check(ctx._lib.b200_mpc_prep_dealer(ctx._h, pk._h, seed & (2**64 - 1), party, parties, C.byref(h)))
+        return MpcPrep(ctx, h)
+
+    def free(self):
+        if self._h:
+            self._ctx._lib.b200_mpc_prep_free(self._ctx._h, self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
+@dataclass
+class MpcResult:
+    proof: B200Proof
+    link_poly_share: np.ndarray   # (n + 2, 4): this party's share of the linking polynomial
+    challenges: np.ndarray        # (6, 4): beta, gamma, alpha, zeta, v, u
+    stats: dict
+
+
+def mpc_last_stats(ctx: Context) -> dict:
+    arr = (C.c_double * 4)()
+    _lib.check(ctx._lib.b200_mpc_last_stats(ctx._h, C.byref(arr)))
+    return {"exchanges": int(arr[0]), "bytes_sent": int(arr[1]), "triples": int(arr[2]), "all_gather_ms": arr[3]}
+
+
+def prove_party(ctx: Context, pk, transport: MpcTransport, prep: MpcPrep, wire_share: np.ndarray, pub_inputs: np.ndarray,
+                blinder_share: np.ndarray) -> MpcResult:
+    """`b200_mpc_prove` for one party over any transport (a caller's, or a LocalGroup's)."""
+    n = pk.domain_size
+    w = np.ascontiguousarray(wire_share, dtype=np.uint64).reshape(5 * n, 4)
+    pi = np.ascontiguousarray(pub_inputs, dtype=np.uint64).reshape(-1, 4)
+    bl = np.ascontiguousarray(blinder_share, dtype=np.uint64).reshape(17, 4)
+    proof = B200Proof()
+    link = np.zeros((n + 2, 4), dtype=np.uint64)
+    ch = np.zeros((6, 4), dtype=np.uint64)
+    vp = lambda a: a.ctypes.data_as(C.c_void_p)
+    _lib.check(ctx._lib.b200_mpc_prove(ctx._h, pk._h, C.byref(transport), prep._h, vp(w), vp(pi) if pi.size else None, vp(bl),
+                                       C.byref(proof), vp(link), vp(ch)))
+    return MpcResult(proof, link, ch, mpc_last_stats(ctx))
+
+
+def _run_parties(fns):
+    """Runs fns[p]() on one thread per party; returns each party's result or the exception it raised."""
+    import threading
+    out = [None] * len(fns)
+
+    def run(p):
+        try:
+            out[p] = fns[p]()
+        except Exception as e:  # noqa: BLE001 - handed back to the caller per party
+            out[p] = e
+
+    ts = [threading.Thread(target=run, args=(p,)) for p in range(len(fns))]
+    for t in ts:
+        t.start()
+    for t in ts:
+        t.join()
+    return out
+
+
+def prove_jointly(ctxs, pks, wire_shares, pub_inputs, blinder_shares, seed: int = 0xBEA7E5, timeout_ms: int = 120000,
+                  transports=None):
+    """All parties of one collaborative proof in this process: one thread per party over a LocalGroup (or over
+    `transports`), dealer preprocessing from `seed`.  Returns every party's MpcResult, or the B200Error it failed with."""
+    P = len(ctxs)
+    group = LocalGroup(P, timeout_ms) if transports is None else None
+    trs = transports if transports is not None else [group.transport(p) for p in range(P)]
+    preps = [MpcPrep.dealer(ctxs[p], pks[p], seed, p, P) for p in range(P)]
+    try:
+        return _run_parties([lambda p=p: prove_party(ctxs[p], pks[p], trs[p], preps[p], wire_shares[p], pub_inputs,
+                                                     blinder_shares[p]) for p in range(P)])
+    finally:
+        for pr in preps:
+            pr.free()
+        if group is not None:
+            group.close()
+
+
+def link_party(ctx: Context, srs: Bases, transport: MpcTransport, a1_share: np.ndarray, a2_share: np.ndarray,
+               comm1: np.ndarray, comm2: np.ndarray, layout):
+    """`b200_mpc_link` for one party: (B200LinkProof, eta)."""
+    from .backend import B200LinkProof
+    a1 = np.ascontiguousarray(a1_share, dtype=np.uint64).reshape(-1, 4)
+    a2 = np.ascontiguousarray(a2_share, dtype=np.uint64).reshape(-1, 4)
+    c1 = np.ascontiguousarray(comm1, dtype=np.uint64).reshape(8)
+    c2 = np.ascontiguousarray(comm2, dtype=np.uint64).reshape(8)
+    proof = B200LinkProof()
+    eta = np.zeros(4, dtype=np.uint64)
+    vp = lambda a: a.ctypes.data_as(C.c_void_p)
+    _lib.check(ctx._lib.b200_mpc_link(ctx._h, srs._h, C.byref(transport), vp(a1), a1.shape[0], vp(a2), a2.shape[0], vp(c1),
+                                      vp(c2), layout.alignment, layout.offset, layout.size, C.byref(proof), vp(eta)))
+    return proof, eta
+
+
+def link_jointly(ctxs, srss, a1_shares, a2_shares, comm1, comm2, layout, timeout_ms: int = 120000):
+    """All parties of one collaborative link proof over a LocalGroup; per party (B200LinkProof, eta) or its B200Error."""
+    P = len(ctxs)
+    group = LocalGroup(P, timeout_ms)
+    trs = [group.transport(p) for p in range(P)]
+    try:
+        return _run_parties([lambda p=p: link_party(ctxs[p], srss[p], trs[p], a1_shares[p], a2_shares[p], comm1, comm2, layout)
+                             for p in range(P)])
+    finally:
+        group.close()

@@ -230,6 +230,11 @@ struct Context {
     // batch verifier (batch_verify.cu): device workspace and the pinned staging of its inputs and results
     DevBuf bv_dev;
     HostPinned bv_host;
+    // collaborative prover (mpc.cu): device workspace, the pinned outgoing message and the P received ones (read by the
+    // kernels through their mapped addresses), and the last call's {exchanges, bytes sent, triples used, ms in all_gather}
+    DevBuf mpc_ws;
+    HostPinned mpc_send, mpc_recv;
+    double mpc_stats[4] = {0, 0, 0, 0};
     ~Context();
 };
 
