@@ -39,6 +39,8 @@ extern "C" {
 #define B200_ERR_NOT_ON_CURVE (-5) /* srs.rs:179 "point not on curve" */
 #define B200_ERR_NO_DEVICE (-6)
 #define B200_ERR_UNSATISFIED (-7)  /* PlonkError::WrongQuotientPolyDegree: witness does not satisfy the circuit */
+#define B200_ERR_MAC (-8)          /* collaborative prover, authenticated shares: the MAC check failed or malformed data was
+                                      received; some party deviated and nothing opened during the call may be used */
 
 typedef struct b200_ctx b200_ctx;     /* one CUDA device + stream + scratch */
 typedef struct b200_bases b200_bases; /* device-resident G1 bases + window tables (the SRS) */
@@ -462,7 +464,7 @@ int b200_fr_poly_div_linear_device(b200_ctx* ctx, const void* d_p, size_t len, c
  * round-2 denominators den r, partial commitments (summed by the library), the five wire evaluations and z(zeta w), the
  * quotient's coefficients above its degree (zero for a satisfied witness), one masked r q[deg], and the transcript state
  * after the verifying key and the public inputs (every party must agree on it, else B200_ERR_INVALID everywhere).
- * Shares are plain additive shares without MACs (semi-honest parties).
+ * Shares are plain additive shares without MACs (semi-honest parties); the authenticated calls below check them.
  * Every message starts with a 32-byte header (exchange index, payload bytes, two zero words), checked on receipt: the
  * wrong exchange or size is B200_ERR_INVALID.  Any failure after the argument checks calls transport->abort. */
 /* all_gather: send `bytes` bytes, receive every party's message in party order (parties * bytes, this party's
@@ -495,7 +497,7 @@ void b200_mpc_prep_free(b200_ctx* ctx, b200_mpc_prep* prep);
 /* wire_shares: 5 x n (host or device pointer), pub_inputs: the key's num_inputs public values (the same on every party),
  * blinder_shares: 17 (draw order of b200_plonk_prove), proof: the opened proof, link_poly_share (n + 2, may be NULL),
  * challenges (6, may be NULL).  Parties on one device may pass the same key.  B200_ERR_UNSATISFIED on every party when
- * the joint witness does not satisfy the circuit. */
+ * the joint witness does not satisfy the circuit.  A preprocessing with MACs (b200_mpc_prep_*_auth) is B200_ERR_INVALID. */
 int b200_mpc_prove(b200_ctx* ctx, const b200_pk* pk, const b200_mpc_transport* transport, b200_mpc_prep* prep,
                    const uint64_t* wire_shares, const uint64_t* pub_inputs, const uint64_t* blinder_shares,
                    b200_proof* proof, uint64_t* link_poly_share, uint64_t* challenges);
@@ -514,9 +516,64 @@ int b200_mpc_local_group_create(int parties, unsigned timeout_ms, b200_mpc_local
 /* The transport of `party`; valid while the group lives. */
 int b200_mpc_local_group_transport(b200_mpc_local_group* group, int party, b200_mpc_transport* out);
 void b200_mpc_local_group_destroy(b200_mpc_local_group* group);
-/* The last b200_mpc_prove / b200_mpc_link on this context: exchanges, bytes sent (headers included), triples used,
- * milliseconds inside all_gather. */
+/* The last b200_mpc_prove / b200_mpc_link / b200_mpc_prove_auth / b200_mpc_link_auth on this context: exchanges, bytes
+ * sent (headers included), triples used, milliseconds inside all_gather. */
 int b200_mpc_last_stats(b200_ctx* ctx, double out[4]);
+
+/* ---- collaborative prover, authenticated shares (device) --------------------------------------------------------
+ * The collaborative prover on SPDZ-style authenticated shares, as ark-mpc's `AuthenticatedScalarResult` and
+ * `CollaborativePlonkProof::open_authenticated` (circuits-core/src/lib.rs:164-177): each party holds a share alpha_i of
+ * a global MAC key alpha (every value Montgomery Fr, 4 limbs), and every shared value x is held as a pair
+ * ([x], [alpha x]).  The calls run the same rounds, Beaver levels and messages as b200_mpc_prove / b200_mpc_link on
+ * both planes; MAC shares are never sent.  Each opened value x_j leaves this party a record
+ * gamma_j = [alpha x_j] - alpha_i x_j.  After the last opening, the parties reveal seeds committed in exchange 0; from
+ * them come rho_s, weighting the records as sigma_i = sum_j gamma_j rho_s^(j+1), and rho_p, combining the MAC planes of
+ * the committed polynomials into one MSM: Sigma_pt,i = MSM(sum_k rho_p^k [alpha p_k]) - alpha_i sum_k rho_p^k C_k.  The
+ * parties commit to (sigma_i, Sigma_pt,i, verdict_i) and reveal them; the call accepts when the sigmas sum to 0, the
+ * points to the identity and every verdict is "accept".  A received field element >= r, or a point off the curve
+ * y^2 = x^3 + 3 or with a coordinate >= q, sets verdict_i = reject; the party still finishes.  So any deviation gives
+ * B200_ERR_MAC on every honest party, and the outputs (proof, challenges, link shares, eta) are written only after the
+ * check passed.  B200_ERR_UNSATISFIED is returned only after the check passed (an unsatisfied witness skips to it).
+ * Security with abort: a deviating party can make the call fail but not make it succeed with a wrong result, except
+ * with probability about (log length + 2) / r per call.
+ *
+ * Messages, against the plain call: exchange 0 carries H(seed_i) (32 bytes) after the 64-byte statement in a proof, and
+ * after the partial quotient commitment in a link; then three more exchanges, each with the 32-byte header:
+ *   seed reveal:   seed_i (32 bytes)
+ *   check commit:  keccak256(record_i) (32 bytes)
+ *   check reveal:  record_i = sigma_i (32) || Sigma_pt,i (64, affine, the identity as zeros) || verdict_i (32: byte 0 is
+ *                  1 for accept, the rest zero) || salt_i (32)  (160 bytes)
+ * H is keccak256.  A proof whose degree check fails skips rounds 4-5, a link whose exactness check fails skips the
+ * opening; both go straight to these exchanges. */
+/* Preprocessing with MACs (the counts of b200_mpc_prep_size): a_mac, b_mac, c_mac, masks_mac are this party's MAC shares
+ * of the triples and masks.  Only b200_mpc_prove_auth accepts it; single use. */
+int b200_mpc_prep_load_auth(b200_ctx* ctx, const b200_pk* pk, const uint64_t* a, const uint64_t* b, const uint64_t* c,
+                            const uint64_t* a_mac, const uint64_t* b_mac, const uint64_t* c_mac, const uint64_t* masks,
+                            const uint64_t* masks_mac, b200_mpc_prep** out);
+/* INSECURE, as b200_mpc_prep_dealer (the same triples and masks for the same seed): alpha and every MAC share are derived
+ * from the seed on the device; mac_key_share receives this party's alpha_i. */
+int b200_mpc_prep_dealer_auth(b200_ctx* ctx, const b200_pk* pk, uint64_t seed, int party, int parties,
+                              uint64_t mac_key_share[4], b200_mpc_prep** out);
+/* INSECURE input stand-in for tests and benchmarks: this party's authenticated shares (shares, macs: count x 4 limbs each)
+ * of `count` values the caller knows in full, under the MAC key b200_mpc_prep_dealer_auth derives from the same seed.
+ * The share masks depend only on (seed, index): two tables shared under one seed get the same masks.  In production
+ * the input protocol of the MPC framework produces these. */
+int b200_mpc_dealer_share_auth(b200_ctx* ctx, uint64_t seed, int party, int parties, const uint64_t* values, size_t count,
+                               uint64_t* shares, uint64_t* macs);
+/* b200_mpc_prove on authenticated shares: wire_macs (5 x n) and blinder_macs (17) are the MAC shares of wire_shares and
+ * blinder_shares; link_poly_mac (n + 2, may be NULL) receives the MAC shares of the linking polynomial.  The opened proof
+ * equals b200_plonk_prove on the summed wires and blinders.  B200_ERR_INVALID for a preprocessing without MACs. */
+int b200_mpc_prove_auth(b200_ctx* ctx, const b200_pk* pk, const b200_mpc_transport* transport, b200_mpc_prep* prep,
+                        const uint64_t* mac_key_share, const uint64_t* wire_shares, const uint64_t* wire_macs,
+                        const uint64_t* pub_inputs, const uint64_t* blinder_shares, const uint64_t* blinder_macs,
+                        b200_proof* proof, uint64_t* link_poly_share, uint64_t* link_poly_mac, uint64_t* challenges);
+/* b200_mpc_link on authenticated hints.  A plaintext hint (a validity proof's) is input by its holder through the MPC
+ * framework's input protocol; "plaintext here, zeros elsewhere" has no valid MACs. */
+int b200_mpc_link_auth(b200_ctx* ctx, const b200_bases* srs, const b200_mpc_transport* transport,
+                       const uint64_t* mac_key_share, const uint64_t* a1_share, const uint64_t* a1_mac, size_t len1,
+                       const uint64_t* a2_share, const uint64_t* a2_mac, size_t len2, const uint64_t* comm1,
+                       const uint64_t* comm2, unsigned alignment, size_t offset, size_t size, b200_link_proof* proof,
+                       uint64_t* eta);
 
 /* ---- witness-side batch hashing (SURVEY.md §8(f) f4) ------------------------------------- */
 /* `batch` independent Poseidon2 sponge hashes of `len` scalars each (inputs: batch x len x 4

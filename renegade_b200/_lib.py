@@ -37,6 +37,8 @@ EXPORTS = [
     "b200_multi_bases_shard", "b200_multi_bases_plan", "b200_multi_msm", "b200_multi_msm_local",
     "b200_mpc_prep_size", "b200_mpc_prep_load", "b200_mpc_prep_dealer", "b200_mpc_prep_free", "b200_mpc_prove", "b200_mpc_link",
     "b200_mpc_local_group_create", "b200_mpc_local_group_transport", "b200_mpc_local_group_destroy", "b200_mpc_last_stats",
+    "b200_mpc_prep_load_auth", "b200_mpc_prep_dealer_auth", "b200_mpc_dealer_share_auth", "b200_mpc_prove_auth",
+    "b200_mpc_link_auth",
 ]
 
 
@@ -184,6 +186,11 @@ def load() -> C.CDLL:
     lib.b200_mpc_local_group_destroy.argtypes = [vp]
     lib.b200_mpc_local_group_destroy.restype = None
     lib.b200_mpc_last_stats.argtypes = [vp, C.POINTER(C.c_double * 4)]
+    lib.b200_mpc_prep_load_auth.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.POINTER(vp)]
+    lib.b200_mpc_prep_dealer_auth.argtypes = [vp, vp, u64, i32, i32, vp, C.POINTER(vp)]
+    lib.b200_mpc_dealer_share_auth.argtypes = [vp, u64, i32, i32, vp, sz, vp, vp]
+    lib.b200_mpc_prove_auth.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.b200_mpc_link_auth.argtypes = [vp, vp, vp, vp, vp, vp, sz, vp, vp, sz, vp, vp, u32, sz, sz, vp, vp]
     lib.b200_keccak256.argtypes = [C.c_char_p, sz, vp]
     lib.b200_keccak256.restype = None
     for name in EXPORTS:

@@ -606,6 +606,15 @@ class MpcPrep:
         _lib.check(ctx._lib.b200_mpc_prep_dealer(ctx._h, pk._h, seed & (2**64 - 1), party, parties, C.byref(h)))
         return MpcPrep(ctx, h)
 
+    @staticmethod
+    def dealer_auth(ctx: Context, pk, seed: int, party: int, parties: int) -> tuple:
+        """INSECURE, as `dealer`, with MACs: (MpcPrep for `prove_party_auth`, this party's MAC-key share as (4,) limbs)."""
+        h = C.c_void_p()
+        key = np.zeros(4, dtype=np.uint64)
+        _lib.check(ctx._lib.b200_mpc_prep_dealer_auth(ctx._h, pk._h, seed & (2**64 - 1), party, parties,
+                                                      key.ctypes.data_as(C.c_void_p), C.byref(h)))
+        return MpcPrep(ctx, h), key
+
     def free(self):
         if self._h:
             self._ctx._lib.b200_mpc_prep_free(self._ctx._h, self._h)
@@ -711,3 +720,120 @@ def link_jointly(ctxs, srss, a1_shares, a2_shares, comm1, comm2, layout, timeout
                              for p in range(P)])
     finally:
         group.close()
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# authenticated shares (b200_mpc_prove_auth / b200_mpc_link_auth): every share x comes with its MAC share [alpha x]
+# ---------------------------------------------------------------------------------------------------------------
+def auth_share_table(values: np.ndarray, parties: int, mac_key_shares, seed: int = 0) -> tuple:
+    """Authenticated additive shares of a (k, 4) table of Montgomery limbs under the MAC key alpha = sum(mac_key_shares)
+    (each a (4,) limb array), in Python integers: (shares, macs), each a list of `parties` (k, 4) tables whose sums are
+    the values and alpha times the values.  For small tables; `dealer_share_auth` does the same on the device."""
+    import random
+    rnd = random.Random(seed)
+    alpha = sum(limbs_to_scalars(np.asarray(k, dtype=np.uint64).reshape(1, 4))[0] for k in mac_key_shares) % R
+    vals = limbs_to_scalars(np.asarray(values, dtype=np.uint64).reshape(-1, 4))
+    shares = [[rnd.randrange(R) for _ in vals] for _ in range(parties - 1)]
+    macs = [[rnd.randrange(R) for _ in vals] for _ in range(parties - 1)]
+    shares.append([(v - sum(col)) % R for v, col in zip(vals, zip(*shares))])
+    macs.append([(alpha * v - sum(col)) % R for v, col in zip(vals, zip(*macs))])
+    return [scalars_to_limbs(s) for s in shares], [scalars_to_limbs(m) for m in macs]
+
+
+def dealer_share_auth(ctx: Context, seed: int, party: int, parties: int, values: np.ndarray) -> tuple:
+    """INSECURE input stand-in (tests, benchmarks): this party's (shares, macs) of a table the caller knows in full,
+    under the MAC key `MpcPrep.dealer_auth` derives from the same seed."""
+    v = np.ascontiguousarray(values, dtype=np.uint64).reshape(-1, 4)
+    sh, mac = np.zeros_like(v), np.zeros_like(v)
+    vp = lambda a: a.ctypes.data_as(C.c_void_p)
+    _lib.check(ctx._lib.b200_mpc_dealer_share_auth(ctx._h, seed & (2**64 - 1), party, parties, vp(v), v.shape[0], vp(sh), vp(mac)))
+    return sh, mac
+
+
+@dataclass
+class MpcAuthResult:
+    proof: B200Proof
+    link_poly_share: np.ndarray   # (n + 2, 4): this party's share of the linking polynomial
+    link_poly_mac: np.ndarray     # (n + 2, 4): its MAC shares
+    challenges: np.ndarray        # (6, 4): beta, gamma, alpha, zeta, v, u
+    stats: dict
+
+
+def prove_party_auth(ctx: Context, pk, transport: MpcTransport, prep: MpcPrep, mac_key_share: np.ndarray, wire_share: np.ndarray,
+                     wire_mac: np.ndarray, pub_inputs: np.ndarray, blinder_share: np.ndarray, blinder_mac: np.ndarray,
+                     proof: B200Proof = None) -> MpcAuthResult:
+    """`b200_mpc_prove_auth` for one party.  `proof` (optional) is the buffer the opened proof is written to; it is
+    left untouched when the call fails."""
+    n = pk.domain_size
+    arr = lambda a, k: np.ascontiguousarray(a, dtype=np.uint64).reshape(k, 4)
+    w, wm = arr(wire_share, 5 * n), arr(wire_mac, 5 * n)
+    bl, blm = arr(blinder_share, 17), arr(blinder_mac, 17)
+    key = arr(mac_key_share, 1)
+    pi = np.ascontiguousarray(pub_inputs, dtype=np.uint64).reshape(-1, 4)
+    proof = B200Proof() if proof is None else proof
+    link, link_mac = np.zeros((n + 2, 4), dtype=np.uint64), np.zeros((n + 2, 4), dtype=np.uint64)
+    ch = np.zeros((6, 4), dtype=np.uint64)
+    vp = lambda a: a.ctypes.data_as(C.c_void_p)
+    _lib.check(ctx._lib.b200_mpc_prove_auth(ctx._h, pk._h, C.byref(transport), prep._h, vp(key), vp(w), vp(wm), vp(pi) if pi.size else None,
+                                            vp(bl), vp(blm), C.byref(proof), vp(link), vp(link_mac), vp(ch)))
+    return MpcAuthResult(proof, link, link_mac, ch, mpc_last_stats(ctx))
+
+
+def prove_jointly_auth(ctxs, pks, wire_values, pub_inputs, blinder_values, seed: int = 0xBEA7E5, timeout_ms: int = 120000,
+                       transports=None, inputs=None, keys=None):
+    """All parties of one authenticated collaborative proof in this process, with dealer preprocessing from `seed`.
+    The wire table and blinders are input with the dealer's MAC key (`dealer_share_auth`), unless `inputs` gives every
+    party's (wire_share, wire_mac, blinder_share, blinder_mac); `keys` may replace the parties' MAC-key shares.  Returns
+    every party's MpcAuthResult, or the B200Error it failed with."""
+    P = len(ctxs)
+    group = LocalGroup(P, timeout_ms) if transports is None else None
+    trs = transports if transports is not None else [group.transport(p) for p in range(P)]
+    made = [MpcPrep.dealer_auth(ctxs[p], pks[p], seed, p, P) for p in range(P)]
+    preps = [m[0] for m in made]
+    keys = keys if keys is not None else [m[1] for m in made]
+    if inputs is None:  # wires and blinders as one table, so that no two values share a mask
+        table = np.concatenate([np.asarray(wire_values, dtype=np.uint64).reshape(-1, 4), np.asarray(blinder_values, dtype=np.uint64).reshape(-1, 4)])
+        k = table.shape[0] - 17
+        inputs = []
+        for p in range(P):
+            sh, mac = dealer_share_auth(ctxs[p], seed, p, P, table)
+            inputs.append((sh[:k], mac[:k], sh[k:], mac[k:]))
+    try:
+        return _run_parties([lambda p=p: prove_party_auth(ctxs[p], pks[p], trs[p], preps[p], keys[p], inputs[p][0], inputs[p][1],
+                                                          pub_inputs, inputs[p][2], inputs[p][3]) for p in range(P)])
+    finally:
+        for pr in preps:
+            pr.free()
+        if group is not None:
+            group.close()
+
+
+def link_party_auth(ctx: Context, srs: Bases, transport: MpcTransport, mac_key_share: np.ndarray, a1_share: np.ndarray,
+                    a1_mac: np.ndarray, a2_share: np.ndarray, a2_mac: np.ndarray, comm1: np.ndarray, comm2: np.ndarray, layout):
+    """`b200_mpc_link_auth` for one party: (B200LinkProof, eta)."""
+    from .backend import B200LinkProof
+    arr = lambda a: np.ascontiguousarray(a, dtype=np.uint64).reshape(-1, 4)
+    a1, a1m, a2, a2m, key = arr(a1_share), arr(a1_mac), arr(a2_share), arr(a2_mac), arr(mac_key_share)
+    c1 = np.ascontiguousarray(comm1, dtype=np.uint64).reshape(8)
+    c2 = np.ascontiguousarray(comm2, dtype=np.uint64).reshape(8)
+    proof = B200LinkProof()
+    eta = np.zeros(4, dtype=np.uint64)
+    vp = lambda a: a.ctypes.data_as(C.c_void_p)
+    _lib.check(ctx._lib.b200_mpc_link_auth(ctx._h, srs._h, C.byref(transport), vp(key), vp(a1), vp(a1m), a1.shape[0], vp(a2), vp(a2m),
+                                           a2.shape[0], vp(c1), vp(c2), layout.alignment, layout.offset, layout.size, C.byref(proof),
+                                           vp(eta)))
+    return proof, eta
+
+
+def link_jointly_auth(ctxs, srss, keys, a1, a2, comm1, comm2, layout, timeout_ms: int = 120000, transports=None):
+    """All parties of one authenticated collaborative link proof; `a1` / `a2` are per-party (share, mac) pairs.  Per
+    party (B200LinkProof, eta) or its B200Error."""
+    P = len(ctxs)
+    group = LocalGroup(P, timeout_ms) if transports is None else None
+    trs = transports if transports is not None else [group.transport(p) for p in range(P)]
+    try:
+        return _run_parties([lambda p=p: link_party_auth(ctxs[p], srss[p], trs[p], keys[p], a1[p][0], a1[p][1], a2[p][0], a2[p][1],
+                                                         comm1, comm2, layout) for p in range(P)])
+    finally:
+        if group is not None:
+            group.close()
